@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py - image-pairs/sec of the OpenGlue matching core on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload C3]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload C3] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
         --master-port P bench.py --gpus N --steps K --warmup W
 
@@ -29,6 +29,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark runs from the built tree and writes nothing into it
 
 import torch  # noqa: E402
 
@@ -36,6 +37,7 @@ from openglue_b200.synthetic import BASELINE_CONFIGS, default_config, synthetic_
 
 METRIC = 'image-pairs/sec at N=M=2048, d=256, 9 GNN layers, 100 Sinkhorn iters'
 MATCH_THRESHOLD = 0.2
+DUMP_BYTES = 60 << 20               # --dump-outputs writes less than 64 MB in all, .npy headers included
 
 
 def flops_per_pair(n, m, d, stages, s):
@@ -126,6 +128,24 @@ def verify_against_fixture(args, res, batch, rank):
     if mism != 0 or err > 3e-4:
         raise SystemExit('bench.py: the timed output does not match the reference fixture: ' + json.dumps(out))
     return out
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: one <out_dir>/<name>.npy per array, float32 kept as float32 and every other dtype stored as float64 (exact
+    for the match indices), so that two builds can be compared output for output on identical inputs.  An array larger than its
+    share of DUMP_BYTES is stored as a fixed sample: its flattened elements at indices drawn by a generator seeded with 0 (sorted,
+    duplicates dropped), with those indices in <name>_sample_index.npy."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    share = DUMP_BYTES // len(arrays)
+    for name, t in arrays.items():
+        t = t.detach()
+        t = t if t.dtype == torch.float32 else t.double()
+        if t.numel() * t.element_size() > share:
+            idx = torch.randint(t.numel(), (share // 16,), generator=torch.Generator().manual_seed(0)).unique()
+            np.save(os.path.join(out_dir, f'{name}_sample_index.npy'), idx.double().numpy())
+            t = t.reshape(-1)[idx.to(t.device)]
+        np.save(os.path.join(out_dir, f'{name}.npy'), t.cpu().numpy())
 
 
 def _numa_nodes():
@@ -297,7 +317,11 @@ def main():
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--no-verify', action='store_true', help='skip the check of the timed output against tests/golden/<workload>_planted.pt')
     ap.add_argument('--cuda-graph', type=int, default=1, help='replay the launch schedule from a CUDA graph (default on)')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help="write rank 0's outputs of the last timed step as DIR/<name>.npy (float32 / float64, under 64 MB in all)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
     wl = dict(BASELINE_CONFIGS[args.workload])
     if args.impl == 'reference':
         return run_reference(args, wl)
@@ -315,11 +339,7 @@ def main():
         dist.init_process_group('nccl', device_id=dev)
 
     from openglue_b200 import _cabi
-    from openglue_b200.build import build
-    if rank == 0:
-        build()
-    if dist is not None:
-        dist.barrier()
+    _cabi.lib()                                # the library build() left in the tree; a missing one is an error
     from openglue_b200.superglue import MatchingCore, SuperGlue
 
     batch = args.pairs_per_gpu or wl['batch']
@@ -400,7 +420,10 @@ def main():
     sampler = ClockSampler(local_rank)
     if rank == 0:
         sampler.start()
-    ms_total = timed(lambda: step(data), args.steps)
+    last = {}
+    ms_total = timed(lambda: last.update(step(data)), args.steps)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, dict(last, loss=loss_acc) if with_loss else last)
     launches = model.last_launches * args.steps
     verified = verify_against_fixture(args, step(data), batch, rank) if not args.no_verify else None
     # ---- end to end through the public API with HOST buffers (H2D + D2H inside the timed region) ----
